@@ -1,6 +1,6 @@
 """bench.py — denoiser steps/sec of the Stage-I temporal-3D-diffusion hot path (BASELINE.json metric) on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--mode temporal|dp]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--mode temporal|dp] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 One "step" = one denoiser step of the default window (SURVEY 8(d), config c2): CFG batch of 2 branches x T=16 frames x
@@ -17,6 +17,8 @@ Prints ONE JSON line (rank 0).
          window per GPU, no collective, weak scaling — BASELINE config 4) the headline instead; either way the other figure
          is reported under `dp` / `temporal_shard`.
 `--impl reference` times the reference's own CPU path (the fp32 oracle port, all host threads) on a fixed bounded sample.
+`--dump-outputs DIR` writes the latents the headline denoise() call returned after its last timed step to DIR/latents.npy
+(fp32, 8 MB).  Weights and inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -202,6 +204,7 @@ def gpu_eager_baseline(dev, steps: int = 3) -> dict:
 
 # ------------------------------------------------------------------------------------------------ B200 arm
 def run_b200(args):
+    import numpy as np
     import torch
     import torch.distributed as dist
 
@@ -278,7 +281,8 @@ def run_b200(args):
         barrier()
         log = ops.event_log
         ops.event_log = None
-        return allmax(ev["t0"].elapsed_time(ev["t1"])), ops.launch_count - marks["launch0"], log, ev["t0"].elapsed_time(ev["t1"])
+        return (allmax(ev["t0"].elapsed_time(ev["t1"])), ops.launch_count - marks["launch0"], log, ev["t0"].elapsed_time(ev["t1"]),
+                lat)
 
     def timed_e2e(host_lat, host_ctx, use_shard):
         """The same metric through the public API with HOST buffers: inputs copied from pinned memory inside the timed region,
@@ -313,7 +317,7 @@ def run_b200(args):
     sampler = ClockSampler(local) if rank == 0 else None
     if temporal_main:
         hl, hc = host_inputs(0)                     # the SAME window on every rank
-        ms_total, launches, log, ms_local = timed_window(hl, hc, True, tags={"attn_self"})  # (few host cycles to spare per launch here)
+        ms_total, launches, log, ms_local, out = timed_window(hl, hc, True, tags={"attn_self"})  # (few host cycles to spare per launch here)
         value = K / (ms_total / 1e3)
         scaling = "strong"
         clocks = sampler.stop() if sampler else None
@@ -321,12 +325,16 @@ def run_b200(args):
         e2e_val = K / (e2e_ms / 1e3)
     else:
         hl, hc = host_inputs(rank)                  # one independent window per GPU
-        ms_total, launches, log, ms_local = timed_window(hl, hc, False, tags={"attn_self", "gemm", "layernorm"})
+        ms_total, launches, log, ms_local, out = timed_window(hl, hc, False, tags={"attn_self", "gemm", "layernorm"})
         value = world * K / (ms_total / 1e3)
         scaling = "weak"
         clocks = sampler.stop() if sampler else None
         e2e_ms, h2d, d2h = timed_e2e(hl, hc, False)
         e2e_val = world * K / (e2e_ms / 1e3)
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "latents.npy"), out.float().cpu().numpy())
+    del out
 
     # ---------------- N > 1: the other multi-GPU figure
     other = None
@@ -334,12 +342,12 @@ def run_b200(args):
         try:
             if temporal_main:
                 hl2, hc2 = host_inputs(rank)
-                ms2, _, _, _ = timed_window(hl2, hc2, False)
+                ms2 = timed_window(hl2, hc2, False)[0]
                 other = ("dp", {"value": world * K / (ms2 / 1e3), "unit": UNIT, "ms_per_step": ms2 / K, "scaling": "weak",
                                 "note": "whole-clip data parallel: one independent window per GPU, no data-path collective"})
             elif shard is not None:
                 hl2, hc2 = host_inputs(0)
-                ms2, _, _, _ = timed_window(hl2, hc2, True)
+                ms2 = timed_window(hl2, hc2, True)[0]
                 other = ("temporal_shard", {"value": K / (ms2 / 1e3), "unit": UNIT, "ms_per_step": ms2 / K, "scaling": "strong",
                                             "frames_per_rank": T // world,
                                             "note": "ONE window, frames sharded over the ranks, temporal-attention K/V all-gathered per layer"})
@@ -530,7 +538,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-video", action="store_true")
     ap.add_argument("--no-eager", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the latents of the last timed step to DIR/latents.npy (B200 path only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to the B200 path")
     if args.impl == "reference":
         run_reference(args, int(os.environ.get("RANK", "0")))
         return

@@ -1,4 +1,4 @@
-"""TEST INFRASTRUCTURE ONLY — regenerate tests/golden/*.pt from the reference's OWN modules (build container only).
+"""TEST INFRASTRUCTURE ONLY — regenerate tests/golden/* from the reference's OWN modules (needs the reference checkout).
 
     python -m oracle.gen_golden
 
@@ -180,8 +180,77 @@ def main():
                 "timesteps": sched.timesteps.clone(), "sigmas": sched.sigmas.clone(), "denoise4_cfg2_out": lat,
                 "state_dict_keys": sorted(tri.state_dict().keys())}, os.path.join(GOLD, "triposg_tiny.pt"))
 
+    reference_outputs(ns, tns)
     for f in sorted(os.listdir(GOLD)):
         print(f, os.path.getsize(os.path.join(GOLD, f)))
+
+
+def _key_paths(node, prefix=""):
+    out = []
+    for k, v in node.items():
+        out.append(prefix + k)
+        if isinstance(v, dict):
+            out += _key_paths(v, prefix + k + ".")
+    return out
+
+
+def reference_outputs(ns, tns):
+    """Fixtures for the tests that compare against the reference's shipped YAML configs, its ImagePreprocessor, a small
+    ActionMeshDenoiser forward + chunk_from, and TripoSG's RectifiedFlowScheduler schedules."""
+    import importlib.util
+    import json
+
+    import numpy as np
+    from PIL import Image
+
+    from actionmesh_b200.config import load_config
+
+    # ---- YAML configs, through the project's own loader: the key tree and the values the B200 presets must keep
+    cdir = os.path.join(reference_loader.REFERENCE_ROOT, "actionmesh", "configs")
+    ref, fast = load_config("actionmesh.yaml", cdir), load_config("actionmesh_fast.yaml", cdir)
+    top = ("stage_0_steps", "face_decimation", "floaters_threshold", "stage_1_steps", "anchor_idx", "sliding_window_denoiser",
+           "subsampling_level", "sliding_window_autoencoder")
+    conf = {"key_paths": sorted(_key_paths(ref)),
+            "values": {k: ref[k] for k in top},
+            "model_blocks": {b: {k: v for k, v in ref.model[b].items() if k != "_target_"} for b in ("scheduler", "cf_guidance")},
+            "fast": {"stage_1_steps": fast.stage_1_steps, "scheduler.num_inference_steps": fast.model.scheduler.num_inference_steps}}
+    with open(os.path.join(GOLD, "reference_config.json"), "w") as f:
+        json.dump(conf, f, indent=1, sort_keys=True)
+        f.write("\n")
+
+    # ---- ImagePreprocessor.process_images (loaded by file path) on the seeded RGBA frames
+    spec = importlib.util.spec_from_file_location(
+        "ref_image_processor", os.path.join(reference_loader.REFERENCE_ROOT, "actionmesh", "preprocessing", "image_processor.py"))
+    ip = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(ip)
+    frames = [Image.fromarray(f, "RGBA") for f in synth.make_rgba_frames()]
+    outs = {}
+    for ind in (False, True):
+        done = ip.ImagePreprocessor(independent_cropping=ind, padding_ratio=0.1).process_images(frames)
+        outs.update({f"independent{int(ind)}_frame{i}": np.asarray(im) for i, im in enumerate(done)})
+    np.savez_compressed(os.path.join(GOLD, "frame_preprocess.npz"), **outs)
+
+    # ---- a 3-layer ActionMeshDenoiser forward (batch of 2, frame 1 observed, no CFG batch); the chunk_from grid
+    d = dict(num_layers=3, num_attention_heads=2, width=256, cross_attention_dim=64, in_channels=64, mlp_ratio=2.0)
+    m = ns.ActionMeshDenoiser(inflated_layers=(0, 1, 2), **d).eval()
+    m.load_state_dict(synth.make_state_dict(m, 9), strict=True)
+    lat, ctx, fs, mask = synth.make_inputs(2, 4, 7, 64, 5, 64, seed=11, observed=(1,))
+    t = torch.tensor([300.0, 300.0])
+    with torch.no_grad():
+        out, _ = m.forward(hidden_states=lat, context=ctx, framestep=fs, diffusion_time=t, mask=mask)
+    chunks = {(start, total): ns.chunk_from(start, total, 16, 15)
+              for total in (16, 17, 31, 32, 47, 64) for start in (0, 3, total // 2, total - 1)}
+    torch.save({"config": d, "seed": 9, "input_seed": 11, "t": t, "forward_out": out,
+                "state_dict_keys": sorted(m.state_dict().keys()), "chunk_from": chunks},
+               os.path.join(GOLD, "denoiser_small3.pt"))
+
+    # ---- TripoSG RectifiedFlowScheduler.set_timesteps
+    sch = {}
+    for n, shift in ((50, 1.0), (100, 3.0), (7, 2.5)):
+        s = tns.RectifiedFlowScheduler(num_train_timesteps=1000, shift=shift)
+        s.set_timesteps(n)
+        sch[(n, shift)] = (s.timesteps.clone(), s.sigmas.clone())
+    torch.save(sch, os.path.join(GOLD, "triposg_schedules.pt"))
 
 
 if __name__ == "__main__":

@@ -1,7 +1,8 @@
-"""TEST INFRASTRUCTURE ONLY.  Import the reference's OWN hot-path modules unchanged from /root/reference.
+"""TEST INFRASTRUCTURE ONLY.  Import the reference's OWN hot-path modules unchanged from a checkout of
+facebookresearch/actionmesh (path in $ACTIONMESH_REFERENCE).
 
-Only usable in the build container (the GPU box has no /root/reference).  Used by gen_golden.py and by the CPU tests
-that pin oracle/denoiser_oracle.py against the reference's code.
+Used only by gen_golden.py, which stores the outputs of these modules under tests/golden/; the tests read those
+fixtures and never need the checkout.
 """
 from __future__ import annotations
 

@@ -68,3 +68,19 @@ def make_inputs(B: int, T: int, N: int, C: int, S: int, Dc: int, seed: int = 5, 
     for o in observed:
         mask[:, o] = 1.0
     return latents, context, framestep, mask
+
+
+def make_rgba_frames(n: int = 5, H: int = 96, W: int = 128, seed: int = 3):
+    """Seeded (H, W, 4) uint8 frames: random RGB under a moving disc of alpha with a soft (partially transparent) edge."""
+    import numpy as np
+
+    rng = np.random.default_rng(seed)
+    out = []
+    for i in range(n):
+        img = rng.integers(0, 256, (H, W, 4), dtype=np.uint8)
+        yy, xx = np.mgrid[0:H, 0:W]
+        cy, cx, r = H // 2 + 3 * i - 4, W // 2 - 2 * i, 20 + 2 * i
+        d = np.sqrt((yy - cy) ** 2 + (xx - cx) ** 2)
+        img[..., 3] = np.clip((r + 6 - d) * 40, 0, 255).astype(np.uint8)
+        out.append(img)
+    return out

@@ -4,6 +4,7 @@ mechanism the reference uses (hydra when installed, else the loader fallback in 
 `defaults:`, `${...}` interpolations resolve, and ActionMeshB200Pipeline keeps the reference's constructor / __call__
 signature (actionmesh/pipeline.py:47-53,602-613) and override plumbing (:637-648)."""
 import inspect
+import json
 import os
 
 import pytest
@@ -11,8 +12,6 @@ import torch
 
 from actionmesh_b200 import AmbError
 from actionmesh_b200.config import DEFAULT_CONFIG_DIR, get_target, instantiate, load_config
-
-REFERENCE_CONFIGS = "/root/reference/actionmesh/configs"
 
 
 def test_default_yaml_resolves_and_instantiates():
@@ -53,10 +52,11 @@ def test_fast_preset_inherits_and_overrides():
     assert cfg2.model.scheduler.num_inference_steps == 4 and list(cfg2.model.cf_guidance.guidance_scales) == [3.0]
 
 
-@pytest.mark.skipif(not os.path.isdir(REFERENCE_CONFIGS), reason="reference checkout not present")
-def test_yaml_keeps_the_reference_keys():
-    """Same key tree as the reference's YAML (only `_target_` values differ), checked with the same loader."""
-    ref = load_config("actionmesh.yaml", REFERENCE_CONFIGS)
+def test_yaml_keeps_the_reference_keys(golden_dir):
+    """Same key tree as the reference's YAML (only `_target_` values differ), checked with the same loader.  The
+    reference side (actionmesh.yaml / actionmesh_fast.yaml loaded by load_config) is stored by oracle/gen_golden.py."""
+    with open(os.path.join(golden_dir, "reference_config.json")) as f:
+        ref = json.load(f)
     ours = load_config("actionmesh_b200.yaml", DEFAULT_CONFIG_DIR)
 
     def keys(node, prefix=""):
@@ -67,17 +67,17 @@ def test_yaml_keeps_the_reference_keys():
                 out |= keys(v, prefix + k + ".")
         return out
 
-    missing = keys(ref) - keys(ours) - {"model.temporal_3D_denoiser.clear_autocast"}  # autocast-cache knob has no meaning here
+    missing = set(ref["key_paths"]) - keys(ours) - {"model.temporal_3D_denoiser.clear_autocast"}  # autocast-cache knob has no meaning here
     assert not missing, missing
-    for k in ("stage_0_steps", "face_decimation", "floaters_threshold", "stage_1_steps", "anchor_idx", "sliding_window_denoiser",
-              "subsampling_level", "sliding_window_autoencoder"):
-        assert ref[k] == ours[k], k
+    assert sorted(ref["values"]) == ["anchor_idx", "face_decimation", "floaters_threshold", "sliding_window_autoencoder",
+                                     "sliding_window_denoiser", "stage_0_steps", "stage_1_steps", "subsampling_level"]
+    for k, v in ref["values"].items():
+        assert ours[k] == v, k
     for blk in ("scheduler", "cf_guidance"):
-        for k, v in ref.model[blk].items():
-            if k != "_target_":
-                assert ours.model[blk][k] == v, (blk, k)
-    fast = load_config("actionmesh_fast.yaml", REFERENCE_CONFIGS)
-    assert fast.stage_1_steps == 15 and fast.model.scheduler.num_inference_steps == 15   # the loader handles `defaults:`
+        assert ref["model_blocks"][blk]
+        for k, v in ref["model_blocks"][blk].items():
+            assert ours.model[blk][k] == v, (blk, k)
+    assert ref["fast"] == {"stage_1_steps": 15, "scheduler.num_inference_steps": 15}   # the loader handles `defaults:`
 
 
 def test_pipeline_signature_and_override_plumbing():

@@ -1,45 +1,23 @@
 """ImagePreprocessor (composite on white, crop to the foreground box, pad to a square) — SURVEY 8(f) rank 3, second half.
 
-CPU: the numpy restatement (oracle/preprocess_oracle.py) against the reference's OWN `ImagePreprocessor.process_images`
-(actionmesh/preprocessing/image_processor.py, loaded by file path; needs only numpy/torch/PIL) when the checkout is present.
+CPU: the numpy restatement (oracle/preprocess_oracle.py) against the outputs of the reference's OWN
+`ImagePreprocessor.process_images` (actionmesh/preprocessing/image_processor.py) on the same seeded frames, stored by
+oracle/gen_golden.py in tests/golden/frame_preprocess.npz.
 GPU (-m gpu): B200FramePreprocessor's uint8 output `array_equal` to the restatement, shared and independent cropping,
 non-square frames, the invalid-alpha error."""
-import importlib.util
 import os
 
 import numpy as np
 import pytest
 
-from oracle import preprocess_oracle
-
-REF = "/root/reference/actionmesh/preprocessing/image_processor.py"
+from oracle import preprocess_oracle, synth
 
 
-def _frames(n=5, H=96, W=128, seed=3):
-    rng = np.random.default_rng(seed)
-    out = []
-    for i in range(n):
-        img = rng.integers(0, 256, (H, W, 4), dtype=np.uint8)
-        yy, xx = np.mgrid[0:H, 0:W]
-        cy, cx, r = H // 2 + 3 * i - 4, W // 2 - 2 * i, 20 + 2 * i
-        d = np.sqrt((yy - cy) ** 2 + (xx - cx) ** 2)
-        alpha = np.clip((r + 6 - d) * 40, 0, 255).astype(np.uint8)       # a disc with a soft (partially transparent) edge
-        img[..., 3] = alpha
-        out.append(img)
-    return out
-
-
-@pytest.mark.skipif(not os.path.exists(REF), reason="reference checkout not present")
 @pytest.mark.parametrize("independent", [False, True])
-def test_restatement_matches_the_reference_module(independent):
-    from PIL import Image
-
-    spec = importlib.util.spec_from_file_location("ref_image_processor", REF)
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    frames = _frames()
-    ref = mod.ImagePreprocessor(independent_cropping=independent, padding_ratio=0.1).process_images(
-        [Image.fromarray(f, "RGBA") for f in frames])
+def test_restatement_matches_the_reference_module(golden_dir, independent):
+    gold = np.load(os.path.join(golden_dir, "frame_preprocess.npz"))
+    frames = synth.make_rgba_frames()
+    ref = [gold[f"independent{int(independent)}_frame{i}"] for i in range(len(frames))]
     ours = preprocess_oracle.frame_preprocess(frames, independent, 0.1)
     assert len(ref) == len(ours)
     for a, b in zip(ref, ours):
@@ -58,14 +36,14 @@ def test_gpu_frame_preprocessing_is_bit_exact(amb_lib, independent):
     from actionmesh_b200.preprocess import B200FramePreprocessor
 
     for H, W in ((96, 128), (130, 70)):
-        frames = _frames(H=H, W=W, seed=H)
+        frames = synth.make_rgba_frames(H=H, W=W, seed=H)
         want = preprocess_oracle.frame_preprocess(frames, independent, 0.1)
         proc = B200FramePreprocessor(independent_cropping=independent, padding_ratio=0.1)
         got = proc.process_images([Image.fromarray(f, "RGBA") for f in frames])
         assert len(got) == len(want)
         for a, b in zip(got, want):
             assert np.array_equal(np.asarray(a), b)
-    bad = _frames(n=1)[0]
+    bad = synth.make_rgba_frames(n=1)[0]
     bad[..., 3] = 255
     with pytest.raises(ValueError):
         B200FramePreprocessor().process_images([Image.fromarray(bad, "RGBA")])

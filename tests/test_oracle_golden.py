@@ -1,12 +1,10 @@
-"""Pins oracle/denoiser_oracle.py (the fp32 restatement that travels to the GPU box) against the golden fixtures that
-oracle/gen_golden.py produced from the reference's OWN modules, and — when /root/reference is present — against those
-modules live.  CPU only."""
-import pytest
+"""Pins oracle/denoiser_oracle.py (the fp32 restatement the GPU tests compare against) against the golden fixtures that
+oracle/gen_golden.py produced from the reference's OWN modules.  CPU only."""
 import torch
 
 from conftest import load_golden
 from oracle import denoiser_oracle as do
-from oracle import reference_loader, synth
+from oracle import synth
 
 
 def _cfg(d):
@@ -98,21 +96,18 @@ def test_stage2_decoder_and_chamfer_match_reference_outputs():
     assert ao.chamfer_score(g["chamfer_a"], g["chamfer_a"], n=0) == 0.0
 
 
-@pytest.mark.skipif(not reference_loader.available(), reason="reference checkout not present (GPU box)")
 def test_oracle_matches_live_reference_modules():
-    ns = reference_loader.load()
-    d = dict(num_layers=3, num_attention_heads=2, width=256, cross_attention_dim=64, in_channels=64, mlp_ratio=2.0)
-    m = ns.ActionMeshDenoiser(inflated_layers=(0, 1, 2), **d).eval()
-    sd = synth.make_state_dict(m, 9)
-    m.load_state_dict(sd, strict=True)  # also pins the state-dict key names of SURVEY A.1
+    """The reference's ActionMeshDenoiser forward on a batch of 2 with an observed frame and no CFG batch, its state-dict
+    key names (SURVEY A.1) and its chunk_from over a grid of window starts, as stored by oracle/gen_golden.py."""
+    g = load_golden("denoiser_small3.pt")
+    d = g["config"]
     cfg = do.DenoiserConfig(inflated_layers=(0, 1, 2), **d)
-    lat, ctx, fs, mask = synth.make_inputs(2, 4, 7, 64, 5, 64, seed=11, observed=(1,))
-    t = torch.tensor([300.0, 300.0])
-    with torch.no_grad():
-        ref, _ = m.forward(hidden_states=lat, context=ctx, framestep=fs, diffusion_time=t, mask=mask)
-    out, _ = do.OracleDenoiser(sd, cfg).forward(lat, ctx, fs, t, mask)
-    assert (out - ref).abs().max() < 2e-5
-    for total in (16, 17, 31, 32, 47, 64):
-        for start in (0, 3, total // 2, total - 1):
-            a, b = ns.chunk_from(start, total, 16, 15), do.chunk_from(start, total, 16, 15)
-            assert len(a) == len(b) and all(torch.equal(x, y) for x, y in zip(a, b))
+    sd = synth.make_state_dict(cfg, g["seed"])
+    assert sorted(sd) == g["state_dict_keys"]
+    lat, ctx, fs, mask = synth.make_inputs(2, 4, 7, 64, 5, 64, seed=g["input_seed"], observed=(1,))
+    out, _ = do.OracleDenoiser(sd, cfg).forward(lat, ctx, fs, g["t"], mask)
+    assert (out - g["forward_out"]).abs().max() < 2e-5
+    assert len(g["chunk_from"]) == 24
+    for (start, total), a in g["chunk_from"].items():
+        b = do.chunk_from(start, total, 16, 15)
+        assert len(a) == len(b) and all(torch.equal(x, y) for x, y in zip(a, b)), (start, total)

@@ -1,12 +1,12 @@
 """Stage 0 (TripoSG DiT + rectified-flow sampler) on the CPU: the oracle restatement and the host-side mirrors against
-the fixture written by the reference's own TripoSGDiTModel / RectifiedFlowScheduler (tests/golden/triposg_tiny.pt,
-oracle/gen_golden.py), plus the live modules when the reference checkout is present."""
+the fixtures written by the reference's own TripoSGDiTModel / RectifiedFlowScheduler (tests/golden/triposg_tiny.pt,
+tests/golden/triposg_schedules.pt, oracle/gen_golden.py)."""
 import pytest
 import torch
 
 from conftest import load_golden
 from oracle import denoiser_oracle as do
-from oracle import reference_loader, synth
+from oracle import synth
 from oracle import triposg_oracle as tro
 
 
@@ -60,14 +60,13 @@ def test_scheduler_mirror_matches_reference_values():
     assert torch.equal(ts[:-1], g["timesteps"]) and torch.allclose(ds, g["sigmas"][:-1] - g["sigmas"][1:])
 
 
-@pytest.mark.skipif(not reference_loader.available(), reason="reference checkout not present")
 def test_live_reference_scheduler_matches_mirror():
+    """Against RectifiedFlowScheduler.set_timesteps of the reference's TripoSG (tests/golden/triposg_schedules.pt)."""
     from actionmesh_b200.stage0 import B200RectifiedFlowScheduler
 
-    ns = reference_loader.load_triposg()
-    for n, shift in ((50, 1.0), (100, 3.0), (7, 2.5)):
-        ref = ns.RectifiedFlowScheduler(num_train_timesteps=1000, shift=shift)
-        ref.set_timesteps(n)
+    ref = load_golden("triposg_schedules.pt")
+    assert sorted(ref) == [(7, 2.5), (50, 1.0), (100, 3.0)]
+    for (n, shift), (ref_timesteps, ref_sigmas) in ref.items():
         ours = B200RectifiedFlowScheduler(num_train_timesteps=1000, shift=shift)
         ours.set_timesteps(n)
-        assert torch.equal(ours.timesteps, ref.timesteps) and torch.equal(ours.sigmas, ref.sigmas)
+        assert torch.equal(ours.timesteps, ref_timesteps) and torch.equal(ours.sigmas, ref_sigmas)
