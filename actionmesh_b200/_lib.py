@@ -10,12 +10,13 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "lib", "libactionmesh_b200.so")
 
-ABI_VERSION = 13
+ABI_VERSION = 14
 
 EXPORTS = [
     "amb_last_error", "amb_abi_version", "amb_device_info", "amb_cfg_euler_step", "amb_layernorm",
     "amb_cast_f32_bf16", "amb_patchify", "amb_timestep_embedding", "amb_alpha_rows", "amb_point_embedding",
-    "amb_displacement_out", "amb_split3_bf16", "amb_softmax_split3", "amb_resize_h_u8", "amb_resize_v_normalize", "amb_alpha_stats", "amb_composite_crop_pad", "amb_nearest_neighbors", "amb_add_bias_rows", "amb_gemm_bf16", "amb_flash_attn_fwd", "amb_attn_small_f32", "amb_debug_set_attn_trace",
+    "amb_displacement_out", "amb_split3_bf16", "amb_softmax_split3", "amb_resize_h_u8", "amb_resize_v_normalize", "amb_alpha_stats", "amb_composite_crop_pad", "amb_nearest_neighbors", "amb_icp_workspace_bytes", "amb_icp_chamfer_grad", "amb_gradient_icp",
+    "amb_transform_points", "amb_add_bias_rows", "amb_gemm_bf16", "amb_flash_attn_fwd", "amb_attn_small_f32", "amb_debug_set_attn_trace",
 ]
 
 
@@ -97,6 +98,13 @@ def load_library() -> C.CDLL:
     lib.amb_alpha_stats.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]
     lib.amb_composite_crop_pad.argtypes = [C.c_void_p] + [C.c_int] * 9 + [C.c_void_p, C.c_void_p]
     lib.amb_nearest_neighbors.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.amb_icp_workspace_bytes.argtypes = [C.c_int, C.c_int, C.c_int, C.POINTER(C.c_size_t)]
+    lib.amb_icp_chamfer_grad.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                         C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.amb_gradient_icp.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
+                                     C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                     C.c_void_p]
+    lib.amb_transform_points.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.amb_patchify.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]
     lib.amb_cast_f32_bf16.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]
     lib.amb_timestep_embedding.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p]

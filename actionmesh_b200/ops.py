@@ -287,6 +287,88 @@ def nearest_neighbors(query: torch.Tensor, reference: torch.Tensor, want_index: 
     return dist, idx
 
 
+ICP_STARTS = 24
+
+
+def adam_tables(lr: float, n_iter: int) -> tuple[torch.Tensor, torch.Tensor]:
+    """torch Adam's per-step scalars in double, as torch.optim.Adam computes them (betas 0.9 / 0.999), rounded to fp32:
+    (lr / (1 - 0.9^t), sqrt(1 - 0.999^t)) for t = 1..n_iter."""
+    step = [lr / (1 - 0.9 ** t) for t in range(1, n_iter + 1)]
+    bc2 = [(1 - 0.999 ** t) ** 0.5 for t in range(1, n_iter + 1)]
+    return torch.tensor(step, dtype=torch.float32), torch.tensor(bc2, dtype=torch.float32)
+
+
+def _icp_inputs(pred: torch.Tensor, gt: torch.Tensor, r_init: torch.Tensor):
+    for t, name in ((pred, "pred"), (gt, "gt"), (r_init, "r_init")):
+        _need(t, torch.float32, name)
+    assert pred.dim() == 3 and pred.shape[2] == 3 and gt.dim() == 3 and gt.shape[2] == 3 and pred.shape[0] == gt.shape[0]
+    assert r_init.shape == (ICP_STARTS, 3, 3)
+    F, P, Q = pred.shape[0], pred.shape[1], gt.shape[1]
+    if F == 0 or P == 0 or Q == 0:
+        raise _lib.AmbError(f"gradient ICP needs non-empty clouds (F={F}, P_pred={P}, P_gt={Q})")
+    nbytes = C.c_size_t()
+    _lib.check(_lib.load_library().amb_icp_workspace_bytes(F, P, Q, C.byref(nbytes)), "amb_icp_workspace_bytes")
+    ws = torch.empty(nbytes.value // 4, dtype=torch.float32, device=pred.device)
+    return pred.contiguous(), gt.contiguous(), r_init.contiguous(), ws, F, P, Q
+
+
+def icp_chamfer_grad(pred: torch.Tensor, gt: torch.Tensor, r_init: torch.Tensor, params: torch.Tensor):
+    """(F, P, 3), (F, Q, 3), (24, 3, 3), params (F, 24, 12) = [r6d | T | s] -> (loss (F, 24), gradient (F, 24, 12)):
+    the Chamfer loss of x = (s * p) @ (r_init[r] @ rot6d(r6d)) + T against gt, and its gradient, per (problem, start)."""
+    global launch_count
+    pred, gt, r_init, ws, F, P, Q = _icp_inputs(pred, gt, r_init)
+    _need(params, torch.float32, "params")
+    assert params.shape == (F, ICP_STARTS, 12)
+    params = params.contiguous()
+    loss = torch.empty(F, ICP_STARTS, dtype=torch.float32, device=pred.device)
+    grad = torch.empty(F, ICP_STARTS, 12, dtype=torch.float32, device=pred.device)
+    rc = _lib.load_library().amb_icp_chamfer_grad(pred.data_ptr(), gt.data_ptr(), F, P, Q, r_init.data_ptr(), params.data_ptr(),
+                                                  ws.data_ptr(), ws.numel() * 4, loss.data_ptr(), grad.data_ptr(), _stream())
+    _lib.check(rc, "amb_icp_chamfer_grad")
+    launch_count += 3
+    return loss, grad
+
+
+def gradient_icp(pred: torch.Tensor, gt: torch.Tensor, r_init: torch.Tensor, lr: float = 0.01, n_iter: int = 200,
+                 want_trace: bool = False):
+    """Batched gradient ICP (actionbench/icp.py:53-112) on the device: (F, P, 3), (F, Q, 3), (24, 3, 3) ->
+    (R (F, 3, 3), T (F, 3), s (F, 3), best loss (F,), best start (F,) int32, loss trace (n_iter, F, 24) or None)."""
+    global launch_count
+    pred, gt, r_init, ws, F, P, Q = _icp_inputs(pred, gt, r_init)
+    if n_iter <= 0:
+        raise _lib.AmbError(f"gradient_icp: n_iter must be positive (got {n_iter})")
+    dev = pred.device
+    step, bc2 = (t.to(dev) for t in adam_tables(lr, n_iter))
+    R = torch.empty(F, 3, 3, dtype=torch.float32, device=dev)
+    T = torch.empty(F, 3, dtype=torch.float32, device=dev)
+    s = torch.empty(F, 3, dtype=torch.float32, device=dev)
+    loss = torch.empty(F, dtype=torch.float32, device=dev)
+    start = torch.empty(F, dtype=torch.int32, device=dev)
+    trace = torch.empty(n_iter, F, ICP_STARTS, dtype=torch.float32, device=dev) if want_trace else None
+    rc = _lib.load_library().amb_gradient_icp(pred.data_ptr(), gt.data_ptr(), F, P, Q, r_init.data_ptr(), n_iter, step.data_ptr(),
+                                              bc2.data_ptr(), ws.data_ptr(), ws.numel() * 4, R.data_ptr(), T.data_ptr(),
+                                              s.data_ptr(), loss.data_ptr(), start.data_ptr(), _ptr(trace), _stream())
+    _lib.check(rc, "amb_gradient_icp")
+    launch_count += 2 + 2 * n_iter
+    return R, T, s, loss, start, trace
+
+
+def transform_points(points: torch.Tensor, R: torch.Tensor, T: torch.Tensor, s: torch.Tensor) -> torch.Tensor:
+    """(F, N, 3) points, per-problem R (F, 3, 3), T (F, 3), s (F, 3) -> (x * s) @ R + T, (F, N, 3)."""
+    global launch_count
+    for t, name in ((points, "points"), (R, "R"), (T, "T"), (s, "s")):
+        _need(t, torch.float32, name)
+    F = points.shape[0]
+    assert points.dim() == 3 and points.shape[2] == 3 and R.shape == (F, 3, 3) and T.shape == (F, 3) and s.shape == (F, 3)
+    points, R, T, s = points.contiguous(), R.contiguous(), T.contiguous(), s.contiguous()
+    out = torch.empty_like(points)
+    rc = _lib.load_library().amb_transform_points(points.data_ptr(), F, points.shape[1], R.data_ptr(), T.data_ptr(), s.data_ptr(),
+                                                  out.data_ptr(), _stream())
+    _lib.check(rc, "amb_transform_points")
+    launch_count += 1
+    return out
+
+
 def cast_bf16(src: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
     global launch_count
     _need(src, torch.float32, "src")

@@ -18,13 +18,14 @@
 #ifndef ACTIONMESH_B200_H_
 #define ACTIONMESH_B200_H_
 
+#include <stddef.h>
 #include <stdint.h>
 
 #ifdef __cplusplus
 extern "C" {
 #endif
 
-#define AMB_ABI_VERSION 13
+#define AMB_ABI_VERSION 14
 
 typedef void* amb_stream_t; /* cudaStream_t */
 
@@ -105,6 +106,34 @@ int amb_composite_crop_pad(const uint8_t* rgba, int n_images, int height, int wi
  * device memory; out_dist / out_index: either may be NULL.  Ties resolve to the lowest index. */
 int amb_nearest_neighbors(const float* query, int n_query, const float* reference, int n_reference, void* scratch_u64,
                           float* out_dist, int32_t* out_index, amb_stream_t stream);
+
+/* Gradient ICP (actionbench/icp.py:53-112, gradient_icp), batched over n_problems cloud pairs x 24 starts.
+ * pred (F, n_pred, 3), gt (F, n_gt, 3) fp32; r_init (24, 3, 3) the canonical start rotations (icp.py:18-49).  Per
+ * (problem f, start r) the parameters are r6d[6], T[3], s[3] (in that order, 12 floats), R = r_init[r] @ rot6d(r6d) and
+ * the prediction moves to x = (s ⊙ p) @ R + T; the loss is pytorch3d's chamfer_distance (mean squared nearest-neighbour
+ * distance, pred->gt plus gt->pred).  Distances are exact fp32 differences; every sum runs in a fixed order, so results
+ * are deterministic and a batch of F problems equals F single calls bit for bit.
+ *  workspace_bytes: device scratch both functions need (amb_icp_workspace_bytes).
+ *  icp_chamfer_grad: params (F, 24, 12) -> out_loss (F, 24) and out_grad (F, 24, 12), the gradient of each start's loss.
+ *  gradient_icp: n_iter iterations of torch's Adam (betas 0.9/0.999, eps 1e-8) on the mean of the 24 losses from r6d =
+ *    (1,0,0,0,1,0), T = 0, s = 1.  step_size / bc2_sqrt: (n_iter) fp32 device tables of lr / (1 - 0.9^t) and
+ *    sqrt(1 - 0.999^t), t = 1..n_iter.  The best start of each problem is tracked like the reference: the first start
+ *    with the minimum loss of an iteration replaces the best only if strictly lower, and the best is stored as the R that
+ *    produced that loss with T and s AFTER that iteration's Adam step (icp.py:96-106).  Outputs: out_rot (F, 3, 3),
+ *    out_t (F, 3), out_s (F, 3), out_loss (F), out_start (F, int32); loss_trace (n_iter, F, 24) may be NULL.
+ *    The host does no work per iteration beyond two kernel launches. */
+int amb_icp_workspace_bytes(int n_problems, int n_pred, int n_gt, size_t* bytes);
+int amb_icp_chamfer_grad(const float* pred, const float* gt, int n_problems, int n_pred, int n_gt, const float* r_init,
+                         const float* params, void* workspace, size_t workspace_bytes, float* out_loss, float* out_grad,
+                         amb_stream_t stream);
+int amb_gradient_icp(const float* pred, const float* gt, int n_problems, int n_pred, int n_gt, const float* r_init,
+                     int n_iter, const float* step_size, const float* bc2_sqrt, void* workspace, size_t workspace_bytes,
+                     float* out_rot, float* out_t, float* out_s, float* out_loss, int32_t* out_start, float* loss_trace,
+                     amb_stream_t stream);
+/* Per-problem transform (pytorch3d Scale(s).compose(Rotate(R), Translate(T)).transform_points):
+ * out[f, i] = points[f, i] @ (diag(s_f) R_f) + T_f; points/out (F, n_points, 3), rot (F, 3, 3), t and s (F, 3). */
+int amb_transform_points(const float* points, int n_problems, int n_points, const float* rot, const float* t,
+                         const float* s, float* out, amb_stream_t stream);
 
 /* ---- Stage II (temporal autoencoder) helpers — first "next" row of SURVEY 8(f) -----------------------------------------
  * alpha_rows: the (source_alpha, target_alpha) token of actionmesh/model/temporal_autoencoder.py:233-237 (TimestepEmbedder,
