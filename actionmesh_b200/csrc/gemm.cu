@@ -674,6 +674,12 @@ extern "C" int amb_gemm_bf16(const amb_gemm_args* a, amb_stream_t stream) {
   AMB_CHECK_ARG(!a->residual || a->ldr % 8 == 0, "gemm: ldr must be a multiple of 8");
   AMB_CHECK_ARG(a->act == 0 || a->act == 1, "gemm: unknown activation %d", a->act);
   AMB_CHECK_ARG(!a->c2 || a->ldc2 % 8 == 0, "gemm: ldc2 must be a multiple of 8");
+  // the epilogue moves 8 columns (bf16) or 4 columns (fp32) per 16-byte access, starting from these base pointers
+  auto al16 = [](const void* q) { return (reinterpret_cast<uintptr_t>(q) & 15) == 0; };
+  AMB_CHECK_ARG(al16(a->c) && al16(a->c2) && al16(a->residual) && al16(a->bias) && al16(a->col_scale),
+                "gemm: c/c2/residual/bias/col_scale must be 16-byte aligned");
+  AMB_CHECK_ARG(al16(a->norm_w0) && al16(a->norm_w1) && al16(a->rope_cos) && al16(a->rope_sin),
+                "gemm: norm weights and rope tables must be 16-byte aligned");
   if (a->norm_cols > 0 || a->rope_cols > 0) {
     AMB_CHECK_ARG(a->n % 128 == 0 && a->norm_cols % 128 == 0 && a->rope_cols % 128 == 0,
                   "gemm: head epilogue needs n, norm_cols, rope_cols multiples of 128");

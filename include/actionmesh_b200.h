@@ -164,7 +164,8 @@ int amb_softmax_split3(const float* scores, int64_t ld_s, int rows, int n, int n
  * a2/k_split), to_q/to_k/to_v with the head split, RMS qk-norm and RoPE of attention_processor.py:92-130 fused in the
  * epilogue, to_out + residual (attention_processor.py:147, block.py:137,146), FeedForward GELU(erf) MLP (block.py:152).
  * A:(m,k) bf16 row-major, W:(n,k) bf16 row-major (nn.Linear layout), fp32 accumulation in TMEM.
- * k % 64 == 0, n % 64 == 0.
+ * k % 64 == 0, n % 64 == 0.  Leading dimensions are multiples of 8 elements; c, c2, residual, bias, col_scale, the
+ * norm weights and the rope tables are 16-byte aligned (the epilogue uses 16-byte loads and stores).
  */
 typedef struct amb_gemm_args {
   const void* a;        /* bf16 (m, k) */
@@ -178,7 +179,8 @@ typedef struct amb_gemm_args {
   int64_t ldc;
   int32_t c_fp32;
   int32_t m, n, k;
-  const float* bias;    /* (n) or NULL */
+  const float* bias;    /* (n) or NULL; not applied to the head columns [0, max(norm_cols, rope_cols)) of the
+                         * RMSNorm/RoPE epilogue, only to the columns past them */
   const void* residual; /* (m', n) bf16/fp32 or NULL; added after the activation; may alias c */
   int64_t ldr;
   int32_t res_fp32;

@@ -73,6 +73,22 @@ def test_argument_validation_fails_loudly(amb_lib):
     g.lda = g.ldw = g.ldc = 64
     rc = amb_lib.amb_gemm_bf16(C.byref(g), None)
     assert rc < 0 and b"multiple of 64" in amb_lib.amb_last_error()
+    # the epilogue's 16-byte loads and stores need 16-byte aligned bases: a bf16 output view at a column offset of 4, or
+    # a misaligned bias / residual / norm / rope pointer, is refused before any tensor map is built
+    g.n = 128
+    for field, bad in (("c", 16 + 8), ("c2", 16 + 4), ("residual", 16 + 2), ("bias", 16 + 4), ("col_scale", 16 + 8)):
+        setattr(g, field, bad)
+        rc = amb_lib.amb_gemm_bf16(C.byref(g), None)
+        assert rc < 0 and b"16-byte aligned" in amb_lib.amb_last_error(), field
+        setattr(g, field, 16 if field == "c" else None)
+    g.norm_cols, g.norm_seg, g.norm_w0 = 128, 128, 16
+    for field in ("norm_w0", "norm_w1", "rope_cos", "rope_sin"):
+        setattr(g, field, 16 + 4)
+        rc = amb_lib.amb_gemm_bf16(C.byref(g), None)
+        assert rc < 0 and b"16-byte aligned" in amb_lib.amb_last_error(), field
+        setattr(g, field, 16 if field == "norm_w0" else None)
+    g.norm_cols = g.norm_seg = 0
+    g.norm_w0 = None
     a = _lib.AttnArgs()
     a.q = a.k = a.v = a.o = 16
     a.batch = a.heads = 1

@@ -113,6 +113,35 @@ def test_flash_attention(probe, name, args, kw):
     assert not res[name]["nan"] and res[name]["rel_fro"] < BF16_REL, res[name]
 
 
+@pytest.mark.parametrize("name,B,H,Sq,Sk,D", [
+    ("d64", 2, 3, 300, 257, 64),
+    ("d128_short_keys", 2, 3, 300, 128 * 7 + 5, 128),     # < 48 key tiles: the single-CTA kernel
+    ("d128_pair", 2, 2, 300, 128 * 48 + 5, 128),          # >= 48 key tiles: the CTA-pair kernel
+])
+def test_flash_attention_output_guard_bands(probe, name, B, H, Sq, Sk, D):
+    """The output is a strided view (rows, heads and head_dim inside a wider buffer) of a buffer prefilled with a NaN
+    sentinel: every element outside the view keeps its bits, with ragged Sq and B, H > 1."""
+    from actionmesh_b200 import ops
+    from oracle import gemm_oracle as go
+
+    g = torch.Generator().manual_seed(11)
+    q = torch.randn(B, Sq, H, D, generator=g).cuda().bfloat16()
+    k = torch.randn(B, Sk, H, D, generator=g).cuda().bfloat16()
+    v = torch.randn(B, Sk, H, D, generator=g).cuda().bfloat16()
+    buf = torch.empty(B, 8 + Sq + 256, H, 32 + D + 64, device="cuda", dtype=torch.bfloat16)
+    buf.view(torch.int16).fill_(go.SENTINEL_BITS[torch.bfloat16])
+    o = buf[:, 8:8 + Sq, :, 32:32 + D]
+    before = buf.clone()
+    ops.flash_attn(q, k, v, o, 1 / math.sqrt(D))
+    torch.cuda.synchronize()
+    written = torch.zeros(buf.shape, dtype=torch.bool, device="cuda")
+    written[:, 8:8 + Sq, :, 32:32 + D] = True
+    assert go.untouched_violations(buf, before, written) == 0
+    ref = probe._attn_ref(q, k, v, 1 / math.sqrt(D))
+    err = float((o.float() - ref).norm() / ref.norm())
+    assert err < BF16_REL and not torch.isnan(o).any(), err
+
+
 def test_flash_attention_late_rescale(probe):
     """Running-max rescale AFTER the first key tile: keys are ordered so that every row's maximum keeps growing by more
     than the lazy-rescale threshold (2^8) along the key axis, with a ragged tail tile."""
